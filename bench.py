@@ -106,6 +106,9 @@ def parse_args():
                     help="N > 1 only: skip the extra timed loop that all-gathers every step's labels over NCCL")
     ap.add_argument("--no-parity-check", action="store_true",
                     help="skip the post-run comparison of one image per arm with the CPU oracle")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the labels and clusters of the last timed step of the headline arm (rank 0) to "
+                         "DIR/<name>.npy, so that two builds can be compared output for output")
     return ap.parse_args()
 
 
@@ -200,6 +203,30 @@ class ClockSampler:
         sm, mx, reasons = parse(inside)
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": sorted(reasons), "samples": len(sm), "scope": scope}
+
+
+DUMP_BYTES = 63_000_000   # array data of --dump-outputs: under 64 MB in all with the .npy headers
+
+
+def dump_outputs(out_dir, labels, clusters):
+    """What the last timed step returned to its caller: labels [B, H, W] (u16 superpixel ids, as float32) and the
+    Cluster records [B, K] (one float64 column per field, in CLUSTER_DTYPE order).  An array larger than its share of
+    DUMP_BYTES is written as a sorted sample of its flat elements (labels) or records (clusters), drawn with a fixed
+    seed, beside the flat indices of the sample as <name>_index.npy."""
+    from fast_slic_b200 import CLUSTER_DTYPE
+    os.makedirs(out_dir, exist_ok=True)
+    B, K = clusters.shape[:2]
+    lab = labels.view(np.uint16).astype(np.float32)
+    cl = np.ascontiguousarray(clusters).reshape(B * K, 32).view(CLUSTER_DTYPE).reshape(-1)
+    rec = np.stack([cl[f].astype(np.float64) for f in CLUSTER_DTYPE.names], -1)
+    for name, a, rows, share in (("labels", lab, lab.reshape(-1), 0.75),
+                                 ("clusters", rec.reshape(B, K, -1), rec, 0.25)):
+        if a.nbytes > share * DUMP_BYTES:
+            n = int(share * DUMP_BYTES // (rows[0].nbytes + 8))
+            idx = np.sort(np.random.RandomState(0).choice(len(rows), n, replace=False))
+            np.save(os.path.join(out_dir, name + "_index.npy"), idx.astype(np.float64))
+            a = rows[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -603,7 +630,7 @@ def main():
     batched = None
     if args.extra_batched > 0 and args.extra_batched != B:
         EB = args.extra_batched
-        nsteps_b = min(200, max(2, pool_steps * B // EB))
+        nsteps_b = args.steps
         flat = pool.view(-1, H, W, 3)
         nb = flat.shape[0] // EB
         if nb >= 1:
@@ -674,7 +701,7 @@ def main():
                 req_submit(i)
             for r_ in req:
                 r_[0].wait()
-            nsteps_s = 4 * nsteps_b
+            nsteps_s = args.steps
             t0s = time.perf_counter()
             for i in range(nsteps_s):
                 req_submit(i)
@@ -700,6 +727,9 @@ def main():
     cpu = None
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         cpu = cpu_reference_run(list(pool.view(-1, H, W, 3)[:8].cpu().numpy()), K, msf, seconds_budget=12.0)
+
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, value_out[1].cpu().numpy(), value_out[2].cpu().numpy())
 
     # ---- parity self-check, outside every timed region: image 0 of the LAST timed step of each arm against the CPU
     # oracle (the compiled reference when oracle/_ref is there).  A fast wrong answer must not print a number.

@@ -1,4 +1,4 @@
-"""CPU-only tests (no GPU in this container): the oracle against the golden vectors and the compiled reference,
+"""CPU-only tests: the oracle against the golden vectors and the compiled reference's recorded answers (conftest.ref),
 the C ABI surface, the host-side logic, and the world_size-2 sharding path over gloo."""
 import ctypes
 import hashlib
@@ -50,7 +50,7 @@ def test_oracle_cca_golden(port, golden):
 
 @pytest.mark.parametrize("case", PIPELINE_CASES[:12], ids=[c[0] for c in PIPELINE_CASES[:12]])
 def test_oracle_matches_compiled_reference(port, ref, case):
-    """Live differential test against oracle/_ref (skipped where the reference sources are not available)."""
+    """Differential test against the compiled reference's answers (conftest.ReferenceAnswers)."""
     name, kind, H, W, K, kw = case
     sigma, a = split_kwargs(kw)
     img = make_image(kind, H, W, seed=13, sigma=sigma)

@@ -1,8 +1,8 @@
 """GPU parity for the exact call patterns bench.py times (VERDICT r1 "what's weak" 1-2): the blocking and the
 streamed HOST entry points at batch 32 (two half uploads, sliced front half, early label download keyed on the
 per-image need_sim flag) and at an odd batch, and several contexts on several streams at once -- every image
-of every step compared with the compiled reference (conftest.Checker falls back to the plain-C restatement
-only where oracle/_ref is absent).  Tolerance 0: labels and raw Cluster bytes.
+of every step compared with the compiled reference's recorded answers (conftest.ReferenceAnswers).  Tolerance 0:
+labels and raw Cluster bytes.
 """
 import numpy as np
 import pytest
