@@ -19,7 +19,7 @@ EXPORTED_SYMBOLS = (
     "fslic_b200_iterate_host_async", "fslic_b200_wait", "fslic_b200_create_cca",
     "fslic_b200_debug_assign_impl", "fslic_b200_connectivity_scratch_bytes", "fslic_b200_get_connectivity",
     "fslic_b200_get_mask_density", "fslic_b200_cluster_density_to_mask", "fslic_b200_cca_stage_ms",
-    "fslic_b200_iterate_real", "fslic_b200_iterate_preemptive",
+    "fslic_b200_iterate_real", "fslic_b200_iterate_preemptive", "fslic_b200_set_manhattan_spatial_dist",
 )
 
 STAGE_NAMES = ("cielab_conversion", "assign", "update", "full_assign", "enforce_connectivity", "iterate")
@@ -78,6 +78,7 @@ def lib():
     L.fslic_b200_get_S.argtypes = [vp]
     L.fslic_b200_launches_last_iterate.argtypes = [vp]
     L.fslic_b200_debug_assign_impl.argtypes = [vp]
+    L.fslic_b200_set_manhattan_spatial_dist.argtypes = [vp, i32]
     L.fslic_b200_connectivity_scratch_bytes.argtypes = [i32]
     L.fslic_b200_connectivity_scratch_bytes.restype = C.c_size_t
     L.fslic_b200_get_connectivity.argtypes = [i32, i32, i32, i32, vp, vp, vp, vp, C.c_size_t, vp]

@@ -3,7 +3,7 @@
 Mirrors /root/reference/fast_slic/base_slic.py:3-62 (BaseSlic / Slic: same kwargs, defaults,
 properties, return dtype) and the Cython ``SlicModel`` (/root/reference/cfast_slic.pyx:15-260,
 attributes cfast_slic.pxd:104-120).  Implemented: the default integer-distance path of the north star, the
-float-distance variants and `preemptive`; LSC raises NotImplementedError.
+float-distance variants, `preemptive` and both spatial metrics (`manhattan_spatial_dist`); LSC raises NotImplementedError.
 """
 import collections
 import contextlib
@@ -71,6 +71,18 @@ def _locked(getter):
         yield eng
     finally:
         eng.lock.release()
+
+
+@contextlib.contextmanager
+def _spatial_metric(eng, manhattan):
+    """Inside a `_locked` block: the context computes with this model's spatial metric for the duration of the call and
+    is handed back with the default (Manhattan) one -- contexts are shared through the cache."""
+    eng.set_manhattan_spatial_dist(manhattan)
+    try:
+        yield eng
+    finally:
+        if not manhattan:
+            eng.set_manhattan_spatial_dist(True)
 
 
 def clear_engine_cache():
@@ -194,12 +206,8 @@ class SlicModel(object):
     def _unsupported(self):
         if self.real_dist and self.real_dist_type not in Engine.REAL_DIST_VARIANTS:
             raise NotImplementedError("real_dist_type %r (LSC) is outside the CUDA hot path" % (self.real_dist_type,))
-        if self.real_dist and self.real_dist_type == "noq" and not self.manhattan_spatial_dist:
-            raise NotImplementedError("SlicRealDistNoQ with manhattan_spatial_dist=False is outside the CUDA hot path")
         if self.preemptive and self.real_dist:
             raise NotImplementedError("preemptive=True together with a float-distance variant is outside the CUDA hot path")
-        if not self.manhattan_spatial_dist:
-            raise NotImplementedError("manhattan_spatial_dist=False is outside the CUDA hot path")
 
     def initialize(self, image):
         """cfast_slic.pyx:124-147."""
@@ -225,7 +233,8 @@ class SlicModel(object):
         clusters = np.ascontiguousarray(self._clusters)[None]
         # the lock covers the timing read-out too: it belongs to this call, not to another thread's next one
         with _locked(lambda: get_engine(H, W, self._num_components, 1, self.device)) as eng:
-            labels = eng.iterate_host(image[None], clusters, params)
+            with _spatial_metric(eng, self.manhattan_spatial_dist):
+                labels = eng.iterate_host(image[None], clusters, params)
             ms = eng.stage_ms()
             cca = eng.cca_stage_ms()
         self._clusters = clusters[0]
@@ -252,10 +261,11 @@ def _iterate_real_dist(self, image, params):
         with torch.cuda.device(eng.device):
             img = torch.from_numpy(image).to(eng.device)[None]
             cl = torch.from_numpy(np.ascontiguousarray(self._clusters).view(np.uint8).reshape(1, -1, 32).copy()).to(eng.device)
-            if self.preemptive:  # cfast_slic.pyx:183-184
-                labels = eng.iterate_preemptive(img, cl, params, self.preemptive_thres)
-            else:
-                labels = eng.iterate_real(self.real_dist_type, img, cl, params)
+            with _spatial_metric(eng, self.manhattan_spatial_dist):
+                if self.preemptive:  # cfast_slic.pyx:183-184
+                    labels = eng.iterate_preemptive(img, cl, params, self.preemptive_thres)
+                else:
+                    labels = eng.iterate_real(self.real_dist_type, img, cl, params)
             ms = eng.stage_ms()
             self._clusters = cl[0].cpu().numpy().view(CLUSTER_DTYPE).reshape(-1)
             out = labels[0].cpu().numpy()
@@ -439,7 +449,7 @@ class BaseSlic(object):
             if images.dtype != np.uint8:
                 raise ValueError("images must be uint8")
         m = self._slic_model
-        with _locked(lambda: get_engine(H, W, K, B, device)) as eng:
+        with _locked(lambda: get_engine(H, W, K, B, device)) as eng, _spatial_metric(eng, m.manhattan_spatial_dist):
             if m.real_dist or m.preemptive:
                 # the float-distance contexts and `preemptive` have device entry points only: host batches go up and down here
                 with torch.cuda.device(eng.device):

@@ -571,14 +571,29 @@ __global__ void __launch_bounds__(256) k_prepare2(PrepParams pp, fslic_cluster* 
 // for di in [-OY, OY], dj in [-OX, OX].  A pixel's entry for candidate c is then at
 //   (i*TS + j) + ((OY - cy)*TS + (OX - cx)):  a per-thread constant plus a per-candidate constant,
 // so the window predicate and both abs() disappear from the inner loop.
+// With manhattan_spatial_dist = false (context.cpp:34-38) the entry is (u16)(coef * hypotf(di, dj)) on the same
+// square window; the kernels that read the table do not change.
 // ---------------------------------------------------------------------------------------------
-__global__ void k_build_sptable(uint16_t* __restrict__ tbl, int S, int OY, int OX, int TS, float coef) {
+
+// glibc's hypotf on integer arguments: it rounds the exact sqrt(a^2 + b^2) once to float, which is what the double
+// square root of the exact double sum gives (a^2 + b^2 < 2^53).  CUDA's hypotf and a float sqrt both differ from it.
+__device__ __forceinline__ float ref_hypotf(int a, int b) {
+    return __double2float_rn(__dsqrt_rn((double)a * (double)a + (double)b * (double)b));
+}
+
+// the reference's u16 spatial term for offsets (di, dj) of the window (context.cpp:30 / :36)
+__device__ __forceinline__ uint32_t spatial_u16(float coef, int di, int dj, int euclid) {
+    const float m = euclid ? ref_hypotf(di, dj) : (float)(abs(di) + abs(dj));
+    return (uint16_t)__float2uint_rz(__fmul_rn(coef, m));
+}
+
+__global__ void k_build_sptable(uint16_t* __restrict__ tbl, int S, int OY, int OX, int TS, float coef, int euclid) {
     const int n = (2 * OY + 1) * TS;
     for (int t = blockIdx.x * blockDim.x + threadIdx.x; t < n; t += gridDim.x * blockDim.x) {
         const int r = t / TS, c = t - r * TS;
         const int di = abs(r - OY), dj = abs(c - OX);
         uint16_t v = (uint16_t)FSLIC_BIGSP;
-        if (di <= S && dj <= S && c <= 2 * OX) v = (uint16_t)__float2uint_rz(__fmul_rn(coef, (float)(di + dj)));
+        if (di <= S && dj <= S && c <= 2 * OX) v = (uint16_t)spatial_u16(coef, di, dj, euclid);
         tbl[t] = v;
     }
 }
@@ -602,6 +617,7 @@ struct AssignParams {
     uint32_t tbl_bytes;             // patch size in shared memory, padded to 128 bytes
     uint32_t cinfo_img_bytes, cells_img_bytes, acc_img_bytes;  // per-image pitches of cinfo / cell_start / acc
     int fuse_prepare;               // 1: the last CTA to finish runs prepare_in_tail for the next pass (small batches)
+    int euclid;                     // manhattan_spatial_dist = false: kernels that compute the spatial term inline use hypotf
 };
 
 #define AS_WARPS 16
@@ -622,9 +638,12 @@ __device__ __forceinline__ void acc_add_pixel(unsigned long long* ac, uint32_t l
 // Brute-force assignment of one pixel straight from the cell grid: lexicographic minimum of
 // (d, phase, k) over the clusters whose window covers (i, j).  Returns the new label (or the kept
 // one) and stores it.  Used by the generic kernel and by warp tiles whose candidate list overflowed.
+// spatial(|di|, |dj|) is the u16 spatial term: computed by the generic kernel, read from the shared patch by the
+// table-driven kernels (which then need neither coef nor the metric in registers).
+template <typename Spatial>
 __device__ __forceinline__ uint32_t assign_pixel_generic(const AssignParams& ap, int i, int j, uint32_t q,
                                                           const CInfo* __restrict__ ci, const int* __restrict__ cs,
-                                                          uint16_t* __restrict__ lb) {
+                                                          uint16_t* __restrict__ lb, Spatial spatial) {
     const int S = ap.S, W = ap.W, H = ap.H;
     unsigned long long best = ~0ull;
     const int cr0 = max(i - S, 0) / ap.G, cr1 = min(i + S, H - 1) / ap.G;
@@ -636,7 +655,7 @@ __device__ __forceinline__ uint32_t assign_pixel_generic(const AssignParams& ap,
             const int cy = (int16_t)(r.cyx & 0xffff), cx = r.cyx >> 16;
             const int di = abs(i - cy), dj = abs(j - cx);
             if (di > S || dj > S) continue;
-            const uint32_t sp = (uint16_t)__float2uint_rz(__fmul_rn(ap.coef, (float)(di + dj)));
+            const uint32_t sp = spatial(di, dj);
             const uint32_t d = sad4_acc(q, r.color, sp) & 0xffffu;  // u16 arithmetic like the scalar reference
             const unsigned long long key = ((unsigned long long)d << 32) | r.sortkey;
             best = key < best ? key : best;
@@ -862,7 +881,9 @@ __global__ void __launch_bounds__(AS_THREADS, AS_MINB) k_assign_warp(AssignParam
                 for (int rr = 0; rr < R; rr++) {
                     if (colok && rr < nrow) {
                         const int i = wi0 + rr * stride;
-                        const uint32_t label = assign_pixel_generic(ap, i, j, q[rr], ci, cs, labels + img_off);
+                        const uint32_t label = assign_pixel_generic(ap, i, j, q[rr], ci, cs, labels + img_off, [&](int di, int dj) {
+                            return (uint32_t)s_tbl[(di + ap.OY) * TS + (dj + ap.OX)];
+                        });
                         if (UPDATE && label != 0xFFFF) acc_add_pixel(ac, label, i, j, q[rr]);
                     }
                 }
@@ -1034,7 +1055,8 @@ __global__ void __launch_bounds__(256) k_assign_generic(AssignParams ap, const u
         const uint32_t q = quad[(size_t)b * ap.H * ap.W + (size_t)i * ap.W + j];
         const uint32_t label = assign_pixel_generic(ap, i, j, q, cinfo + (size_t)b * ap.K,
                                                     cell_start + (size_t)b * (ap.ncell + 1),
-                                                    labels + (size_t)b * ap.H * ap.W);
+                                                    labels + (size_t)b * ap.H * ap.W,
+                                                    [&](int di, int dj) { return spatial_u16(ap.coef, di, dj, ap.euclid); });
         if (UPDATE && label != 0xFFFF) acc_add_pixel(acc + (size_t)b * ap.K * 4, label, i, j, q);
     }
 }

@@ -310,7 +310,9 @@ __global__ void __launch_bounds__(32 * A5_MAXWARPS, 1)
                 for (int rr = 0; rr < R; rr++) {
                     if (j < W && rr < nrow) {
                         const int i = wi0 + rr * stride;
-                        const uint32_t label = assign_pixel_generic(ap, i, j, q[rr], ci, cs, labels + img_off);
+                        const uint32_t label = assign_pixel_generic(ap, i, j, q[rr], ci, cs, labels + img_off, [&](int di, int dj) {
+                            return lds_u16(sbase + 2u * (uint32_t)((di + ap.OY) * TS + (dj + ap.OX)));
+                        });
                         if (UPDATE && label != 0xFFFF) acc_add_pixel(ac, label, i, j, q[rr]);
                     }
                 }

@@ -137,7 +137,8 @@ struct fslic_ctx {
         const void *img, *cl, *lab;
         int batch;
         fslic_params p;
-    } gkey = {nullptr, nullptr, nullptr, 0, {0.f, 0.f, 0, 0, 0, 0}}, gkey_seen = {nullptr, nullptr, nullptr, 0, {0.f, 0.f, 0, 0, 0, 0}};
+        int manhattan;  // the spatial metric is baked into the captured kernels' parameters
+    } gkey = {nullptr, nullptr, nullptr, 0, {0.f, 0.f, 0, 0, 0, 0}, 1}, gkey_seen = {nullptr, nullptr, nullptr, 0, {0.f, 0.f, 0, 0, 0, 0}, 1};
     int glaunches = 0;
     float assign_kernel_ms = 0.f;
     int assign_kernel_launches = 0;
@@ -145,6 +146,10 @@ struct fslic_ctx {
     int spt_stride = 0;
     cudaStream_t spt_stream = nullptr;
     uint32_t spt_coef_bits = 0;
+    bool spt_manhattan = true;
+    // the reference's public context field manhattan_spatial_dist (context.h:35): L1 (default) or Euclidean spatial term;
+    // read by every entry point when it enqueues work (fslic_b200_set_manhattan_spatial_dist)
+    bool manhattan = true;
     int assign_impl = 5;       // 5: TMA-staged kernel where it applies (default), 4: always the LDG kernel (FSLIC_ASSIGN=4)
     int last_assign_impl = 0;  // which kernel the last subsampled / full pass used (tests, bench)
 };
@@ -155,6 +160,11 @@ extern "C" int fslic_b200_sizeof_cluster(void) { return (int)sizeof(fslic_cluste
 extern "C" int fslic_b200_get_S(const fslic_ctx* ctx) { return ctx ? ctx->S : -1; }
 extern "C" int fslic_b200_launches_last_iterate(const fslic_ctx* ctx) { return ctx ? ctx->last_launches : -1; }
 extern "C" int fslic_b200_debug_assign_impl(const fslic_ctx* ctx) { return ctx ? ctx->last_assign_impl : -1; }
+extern "C" int fslic_b200_set_manhattan_spatial_dist(fslic_ctx* ctx, int manhattan) {
+    if (!ctx) return set_err(FSLIC_EINVAL, "ctx is NULL");
+    ctx->manhattan = manhattan != 0;
+    return FSLIC_OK;
+}
 
 // ---- Lab tables: FastCIELabCvt ctor, /root/reference/src/cielab.h:297-305 ----------------------
 // _srgb_gamma_tbl (cielab.h:22-279) is the sRGB inverse companding curve documented at
@@ -680,7 +690,7 @@ static bool make_subrow_map(CUtensorMap* m, CUtensorMapDataType dt, int esize, v
 }
 
 static int build_patches(fslic_ctx* c, int stride, bool need_sub, float coef, cudaStream_t st, int* launches) {
-    // The two patches depend on (S, stride, coef) only: consecutive calls with the same parameters reuse them (two
+    // The two patches depend on (S, stride, coef, metric) only: consecutive calls with the same parameters reuse them (two
     // launches less per call, four on the sliced host path).  Inside a stream capture they are always rebuilt, so a
     // replayed graph never depends on what an unrelated call left in the buffers.
     cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
@@ -688,23 +698,24 @@ static int build_patches(fslic_ctx* c, int stride, bool need_sub, float coef, cu
     uint32_t coef_bits;
     memcpy(&coef_bits, &coef, 4);
     const bool warm = cap == cudaStreamCaptureStatusNone && c->spt_valid && c->spt_stream == st && c->spt_stride == stride &&
-                      c->spt_coef_bits == coef_bits && (c->spt_has_sub || !need_sub);
+                      c->spt_coef_bits == coef_bits && c->spt_manhattan == c->manhattan && (c->spt_has_sub || !need_sub);
     if (warm) return FSLIC_OK;
     c->spt_valid = true;
     c->spt_stream = st;  // a call on another stream is not ordered after this build: it rebuilds
     c->spt_stride = stride;
     c->spt_coef_bits = coef_bits;
+    c->spt_manhattan = c->manhattan;
     c->spt_has_sub = need_sub;
     if (need_sub) {
         const PassGeom g = pass_geometry(c, stride);
         if (g.fast) {
-            k_build_sptable<<<64, 256, 0, st>>>(c->sptable, c->S, g.OY, g.OX, g.TS, coef);
+            k_build_sptable<<<64, 256, 0, st>>>(c->sptable, c->S, g.OY, g.OX, g.TS, coef, !c->manhattan);
             if (launches) *launches += 1;
         }
     }
     const PassGeom gf = pass_geometry(c, 1);
     if (gf.fast) {
-        k_build_sptable<<<64, 256, 0, st>>>(c->sptable + SPT_MAX_ELEMS, c->S, gf.OY, gf.OX, gf.TS, coef);
+        k_build_sptable<<<64, 256, 0, st>>>(c->sptable + SPT_MAX_ELEMS, c->S, gf.OY, gf.OX, gf.TS, coef, !c->manhattan);
         if (launches) *launches += 1;
     }
     CK(cudaGetLastError());
@@ -728,6 +739,7 @@ static int run_assign_pass(fslic_ctx* c, int batch, int stride, int rem, int cfg
         ap.cfg_stride = cfg_stride; ap.fresh_from = fresh_from;
         ap.G = c->G; ap.cellW = c->cellW; ap.cellH = c->cellH; ap.ncell = c->ncell;
         ap.coef = coef;
+        ap.euclid = !c->manhattan;
         const long px = (long)ap.nsub * c->W * batch;
         long grid = (px + 255) / 256;
         if (grid > (long)c->num_sms * 32) grid = (long)c->num_sms * 32;
@@ -751,6 +763,7 @@ static int run_assign_pass(fslic_ctx* c, int batch, int stride, int rem, int cfg
         ap.cfg_stride = cfg_stride; ap.fresh_from = fresh_from;
         ap.G = c->G; ap.cellW = c->cellW; ap.cellH = c->cellH; ap.ncell = c->ncell;
         ap.coef = coef;
+        ap.euclid = !c->manhattan;
         const long px = (long)ap.nsub * c->W * batch;
         long grid = (px + 255) / 256;
         if (grid > (long)c->num_sms * 32) grid = (long)c->num_sms * 32;
@@ -781,6 +794,7 @@ static int run_assign_pass(fslic_ctx* c, int batch, int stride, int rem, int cfg
     ap.tiles_y = ceil_div(ap.nsub, g.R);
     ap.ntiles = ap.tiles_x * ap.tiles_y;
     ap.coef = coef;
+    ap.euclid = !c->manhattan;
     ap.tps = AS_T;
     ap.fuse_prepare = 0;
     // The TMA-staged kernel: row strides of the tensor maps must be multiples of 16 bytes (W % 8 == 0 for the u16
@@ -967,7 +981,8 @@ static int run_prepare(fslic_ctx* c, fslic_cluster* d_clusters, int batch, int f
     return FSLIC_OK;
 }
 
-static int check_params(const fslic_ctx* c, const fslic_params* p, float* coef_out) {
+// variant: as in iterate_front (-1 the default integer path); ContextRealDistL2 (1) keeps its squared term whatever the flag
+static int check_params(const fslic_ctx* c, const fslic_params* p, float* coef_out, int variant = -1) {
     if (!p) return set_err(FSLIC_EINVAL, "params is NULL");
     if (p->subsample_stride <= 0 || p->subsample_stride > 255) return set_err(FSLIC_EINVAL, "subsample_stride must be in 1..255");
     if (p->max_iter < 0) return set_err(FSLIC_EINVAL, "max_iter must be >= 0");
@@ -977,7 +992,9 @@ static int check_params(const fslic_ctx* c, const fslic_params* p, float* coef_o
     // BaseContext::set_spatial_patch, context.cpp:25-26 (same float operations, same order)
     float coef = 1.0f / ((float)S / p->compactness);
     coef *= (float)(1 << color_shift);
-    if (S > 0 && !(coef * (float)(2 * S) < (float)(FSLIC_BIGSP - 766)))
+    // the largest patch value: coef * 2S (Manhattan), coef * hypotf(S, S) (Euclidean, context.cpp:36)
+    const float reach = (!c->manhattan && variant != 1) ? (float)sqrt(2.0 * (double)S * (double)S) : (float)(2 * S);
+    if (S > 0 && !(coef * reach < (float)(FSLIC_BIGSP - 766)))
         return set_err(FSLIC_ERANGE, "compactness too large: the u16 distance of the reference would overflow");
     if (S == 0) coef = 0.f;  // 1/(0/compactness) = inf in the reference; with S == 0 only m = 0 is ever used -> inf*0 = NaN -> (u16) UB; use 0
     *coef_out = coef;
@@ -1041,7 +1058,7 @@ static int iterate_plain(fslic_ctx* c, const uint8_t* d_images, fslic_cluster* d
     int rc = check_batch(c, batch);
     if (rc) return rc;
     float coef;
-    rc = check_params(c, p, &coef);
+    rc = check_params(c, p, &coef, variant);
     if (rc) return rc;
     USE_DEVICE(c->device);
     cudaStream_t st = (cudaStream_t)stream;
@@ -1099,7 +1116,7 @@ extern "C" int fslic_b200_iterate(fslic_ctx* c, const uint8_t* d_images, fslic_c
     if (c && p && c->graphs_enabled && batch > 0 && batch < 4 && p->collect_timing == 0 && stream != nullptr) {
         fslic_ctx::GraphKey k;
         memset(&k, 0, sizeof(k));
-        k.img = nullptr; k.cl = d_clusters; k.lab = d_labels; k.batch = batch; k.p = *p;
+        k.img = nullptr; k.cl = d_clusters; k.lab = d_labels; k.batch = batch; k.p = *p; k.manhattan = c->manhattan;
         const bool have = c->gexec && memcmp(&k, &c->gkey, sizeof(k)) == 0;
         const bool again = memcmp(&k, &c->gkey_seen, sizeof(k)) == 0;
         memcpy(&c->gkey_seen, &k, sizeof(k));
@@ -1109,7 +1126,7 @@ extern "C" int fslic_b200_iterate(fslic_ctx* c, const uint8_t* d_images, fslic_c
 }
 
 // The float-distance contexts of the reference (context.h:100-125; cfast_slic.pyx:198-252): variant 0 = ContextRealDist
-// ("standard"), 1 = ContextRealDistL2, 2 = ContextRealDistNoQ with manhattan_spatial_dist (its default).
+// ("standard"), 1 = ContextRealDistL2, 2 = ContextRealDistNoQ; the spatial metric is the context's manhattan flag.
 extern "C" int fslic_b200_iterate_real(fslic_ctx* c, int variant, const uint8_t* d_images, fslic_cluster* d_clusters,
                                        uint16_t* d_labels, int batch, const fslic_params* p, void* stream) {
     if (variant < 0 || variant > 2) return set_err(FSLIC_EINVAL, "variant must be 0 (standard), 1 (l2) or 2 (noq)");
@@ -1236,7 +1253,7 @@ static int iterate_graphed(fslic_ctx* c, const uint8_t* d_images, fslic_cluster*
     if (rc) return rc;
     fslic_ctx::GraphKey k;
     memset(&k, 0, sizeof(k));
-    k.img = nullptr; k.cl = d_clusters; k.lab = d_labels; k.batch = batch; k.p = *p;
+    k.img = nullptr; k.cl = d_clusters; k.lab = d_labels; k.batch = batch; k.p = *p; k.manhattan = c->manhattan;
     {
         USE_DEVICE(c->device);
         c->slice = 0;

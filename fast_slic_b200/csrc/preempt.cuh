@@ -94,7 +94,7 @@ __global__ void __launch_bounds__(256) k_assign_preempt(AssignParams ap, const u
                 const int di = abs(i - cy), dj = abs(j - cx);
                 if (di > S || dj > S) continue;
                 if (!cl[rec.sortkey & 0xffffu].is_active) continue;  // context.cpp:218
-                const uint32_t sp = (uint16_t)__float2uint_rz(__fmul_rn(ap.coef, (float)(di + dj)));
+                const uint32_t sp = spatial_u16(ap.coef, di, dj, ap.euclid);
                 const uint32_t d = sad4_acc(q, rec.color, sp) & 0xffffu;
                 const unsigned long long key = ((unsigned long long)d << 32) | rec.sortkey;
                 best = key < best ? key : best;

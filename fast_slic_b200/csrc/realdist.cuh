@@ -10,6 +10,10 @@
 //   VARIANT 0  d = coef * (|di| + |dj|)  +  (|dr| + |dg| + |db|)                     one multiply, one add
 //   VARIANT 1  d = fma(dj', dj', di' * di')  +  (dr^2 + dg^2 + db^2),  di' = coef * di   (GCC fuses the patch like this)
 //   VARIANT 2  d = |r - cr| + |g - cg| + |b - cb| + |coef (j - cx)| + |coef (i - cy)|  on float centroids, left to right
+// With manhattan_spatial_dist = false (AssignParams.euclid; context.cpp:34-38, :488-491):
+//   VARIANT 0  the patch is coef * hypotf(di, dj)
+//   VARIANT 1  unchanged: ContextRealDistL2::set_spatial_patch ignores the flag
+//   VARIANT 2  d = fma(dx, dx, fma(db, db, fma(dr, dr, dg * dg))) + dy * dy   (the -mfma object code: dy^2 once per row)
 // Ties: strict '>' against the running minimum in visiting order => minimum of (d, phase, k); non-negative floats
 // order like their bit patterns, so the key is  float_bits(d) << 32 | phase << 16 | k.
 #pragma once
@@ -53,14 +57,22 @@ __global__ void __launch_bounds__(256) k_assign_real(AssignParams ap, const uint
                     if (i < i0 || i >= i1 || j < j0 || j >= j1) continue;
                     const float dr = __fsub_rn((float)qr, c.r), dg = __fsub_rn((float)qg, c.g), db = __fsub_rn((float)qb, c.b);
                     const float dy = __fmul_rn(coef, __fsub_rn((float)i, c.y)), dx = __fmul_rn(coef, __fsub_rn((float)j, c.x));
-                    d = __fadd_rn(__fadd_rn(__fadd_rn(__fadd_rn(fabsf(dr), fabsf(dg)), fabsf(db)), fabsf(dx)), fabsf(dy));
+                    if (ap.euclid) {  // assign_clusters_proto<false>, context.cpp:490, as its -mfma object code evaluates it
+                        float t = __fmul_rn(dg, dg);
+                        t = __fmaf_rn(dr, dr, t);
+                        t = __fmaf_rn(db, db, t);
+                        t = __fmaf_rn(dx, dx, t);
+                        d = __fadd_rn(t, __fmul_rn(dy, dy));
+                    } else {
+                        d = __fadd_rn(__fadd_rn(__fadd_rn(__fadd_rn(fabsf(dr), fabsf(dg)), fabsf(db)), fabsf(dx)), fabsf(dy));
+                    }
                 } else {
                     const int cy = (int16_t)(r.cyx & 0xffff), cx = r.cyx >> 16;
                     const int di = i - cy, dj = j - cx;
                     if (abs(di) > S || abs(dj) > S) continue;
                     const int cr_ = r.color & 0xff, cg_ = (r.color >> 8) & 0xff, cb_ = (r.color >> 16) & 0xff;
                     if (VARIANT == 0) {
-                        const float patch = __fmul_rn(coef, (float)(abs(di) + abs(dj)));
+                        const float patch = __fmul_rn(coef, ap.euclid ? ref_hypotf(di, dj) : (float)(abs(di) + abs(dj)));
                         d = __fadd_rn(patch, (float)(abs(qr - cr_) + abs(qg - cg_) + abs(qb - cb_)));
                     } else {
                         const float fdi = __fmul_rn(coef, (float)di), fdj = __fmul_rn(coef, (float)dj);

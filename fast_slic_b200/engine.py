@@ -80,6 +80,11 @@ class Engine:
         return Params(float(compactness), float(min_size_factor), int(subsample_stride), int(bool(convert_to_lab)),
                       int(max_iter), int(collect_timing))
 
+    def set_manhattan_spatial_dist(self, manhattan):
+        """The spatial term of every later iterate call: L1 (True, the default) or Euclidean (False), like the reference's
+        context field manhattan_spatial_dist.  It is context state: callers sharing a context set it under `lock`."""
+        check(self._L.fslic_b200_set_manhattan_spatial_dist(self._h, int(bool(manhattan))))
+
     # -- device entry points -------------------------------------------------------------------
     def initialize_clusters(self, images, clusters=None):
         self._check_images(images)

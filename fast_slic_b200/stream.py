@@ -7,7 +7,9 @@ on the same images (every batch is a cold start from the grid seeding, like a fr
 
 `warm_start=True` is the reference's video use (README.md:3; cfast_slic.pyx:160 keeps `_c_clusters` between calls):
 image b of every batch is the next frame of stream b and starts from the clusters its previous frame ended with --
-exactly what calling `slic.iterate(frame)` again on the same `Slic` object does.  Frame t+1 of a stream depends on
+exactly what calling `slic.iterate(frame)` again on the same `Slic` object does.
+
+`manhattan_spatial_dist=False` selects the Euclidean spatial term, like the keyword of `Slic`.  Frame t+1 of a stream depends on
 the clusters of frame t, so in this mode a submit waits for the previous batch to finish (its clusters are the
 input); the upload of the new frames is still prepared while the previous batch computes.
 """
@@ -34,12 +36,16 @@ class _Slot:
 
 class SlicStream:
     def __init__(self, height, width, num_components, batch, depth=2, device=0, compactness=10.0,
-                 min_size_factor=0.25, subsample_stride=3, convert_to_lab=True, max_iter=10, warm_start=False):
+                 min_size_factor=0.25, subsample_stride=3, convert_to_lab=True, max_iter=10, warm_start=False,
+                 manhattan_spatial_dist=True):
         require_cuda()
         if depth < 1:
             raise ValueError("depth must be >= 1")
         self.H, self.W, self.K, self.batch = int(height), int(width), int(num_components), int(batch)
         self._slots = [_Slot(self.H, self.W, self.K, self.batch, device) for _ in range(depth)]
+        self.manhattan_spatial_dist = bool(manhattan_spatial_dist)
+        for s in self._slots:  # the slots' contexts are this stream's own: the metric is set once
+            s.engine.set_manhattan_spatial_dist(self.manhattan_spatial_dist)
         self._params = self._slots[0].engine.params(compactness, min_size_factor, subsample_stride, convert_to_lab,
                                                     max_iter)
         self._free = collections.deque(self._slots)

@@ -51,7 +51,8 @@ enum {
     FSLIC_EINVAL = -1,   /* bad argument (reference: ValueError, cfast_slic.pyx:24-27,125,153) */
     FSLIC_ECUDA = -2,    /* CUDA runtime error */
     FSLIC_ENOMEM = -3,
-    FSLIC_ERANGE = -4    /* compactness so large the u16 distance would overflow (UB in the reference) */
+    FSLIC_ERANGE = -4    /* compactness so large the u16 distance would overflow (UB in the reference); bounded by the
+                            largest patch value of the metric in use */
 };
 
 typedef struct fslic_ctx fslic_ctx;
@@ -79,6 +80,12 @@ int fslic_b200_destroy(fslic_ctx* ctx);
  *    K (max_label_size) is an argument of that call, exactly like the reference's constructor argument. */
 int fslic_b200_create_cca(int device, int H, int W, int max_batch, fslic_ctx** out);
 
+/* == the public context field `manhattan_spatial_dist` (context.h:35; cfast_slic.pyx:186,246): nonzero (the default) for
+ *    the L1 spatial term coef * (|di| + |dj|), 0 for the Euclidean coef * hypotf(di, dj) of classic SLIC
+ *    (context.cpp:23-40, :462-499).  Every iterate entry point reads it when it enqueues work; a call already enqueued
+ *    keeps the metric it was enqueued with. */
+int fslic_b200_set_manhattan_spatial_dist(fslic_ctx* ctx, int manhattan);
+
 /* == BaseContext::initialize_clusters (context.cpp:43-97), for `batch` images [B,H,W,3] u8. */
 int fslic_b200_initialize_clusters(fslic_ctx* ctx, const uint8_t* d_images, fslic_cluster* d_clusters, int batch,
                                    void* stream);
@@ -92,9 +99,10 @@ int fslic_b200_iterate(fslic_ctx* ctx, const uint8_t* d_images, fslic_cluster* d
 /* == the float-distance contexts ContextRealDist / ContextRealDistL2 / ContextRealDistNoQ (context.h:100-125,
  *    context.cpp:394-499; selected in cfast_slic.pyx:198-252 by SlicModel.real_dist_type): `variant` 0 = "standard"
  *    (the default kernel with float distances and an untruncated float spatial term), 1 = "l2" (squared colour and
- *    spatial distances), 2 = "noq" (float centroids, no quantisation in the update; Manhattan spatial term, the
- *    reference's default).  Same buffers and semantics as fslic_b200_iterate; results bit-identical to the reference
- *    (every float operation in its order and rounding). */
+ *    spatial distances), 2 = "noq" (float centroids, no quantisation in the update).  The spatial term follows
+ *    fslic_b200_set_manhattan_spatial_dist, except for "l2", whose squared term ignores it (context.cpp:435-445).  Same
+ *    buffers and semantics as fslic_b200_iterate; results bit-identical to the reference (every float operation in its
+ *    order and rounding). */
 int fslic_b200_iterate_real(fslic_ctx* ctx, int variant, const uint8_t* d_images, fslic_cluster* d_clusters,
                             uint16_t* d_labels, int batch, const fslic_params* params, void* stream);
 
